@@ -6,11 +6,13 @@ lighting + HDR post chain on a 3840x2160 synthetic G-buffer with 4096 lights (BA
   python bench.py --impl reference --gpus N --steps K ...  # the reference's algorithm on the host cores
                                                            # (CPU oracle; the reference has no CPU path
                                                            #  and no Vulkan device exists here)
-Prints ONE JSON line on rank 0.  A "step" is one frame.
+Prints ONE JSON line on rank 0.  A "step" is one frame.  --dump-outputs DIR writes the output frame of
+the last timed step as .npy files, so that two builds can be compared on the same seeded inputs.
 """
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import math
 import os
@@ -52,6 +54,22 @@ def algorithmic_bytes(w, h, aa, bloom=True):
     return lighting, chain, total
 
 
+DUMP_PIXELS = 1 << 21  # a larger frame is dumped as this many pixels, a seeded sample: 48 MB with their indices
+
+
+def dump_outputs(out_dir, frame):
+    """Writes the RGBA8 output frame (rows, width) uint32 as out_dir/frame_rgba8.npy: float32 (rows, width, 4)
+    of the 0..255 channel values, or, above DUMP_PIXELS pixels, float32 (DUMP_PIXELS, 4) for a fixed seeded
+    sample of them plus out_dir/frame_rgba8_index.npy, their row-major pixel indices as float64."""
+    os.makedirs(out_dir, exist_ok=True)
+    rgba = np.ascontiguousarray(frame).view(np.uint8).reshape(frame.shape[0], frame.shape[1], 4).astype(np.float32)
+    if frame.size > DUMP_PIXELS:
+        idx = np.sort(np.random.default_rng(0).choice(frame.size, DUMP_PIXELS, replace=False))
+        rgba = rgba.reshape(-1, 4)[idx]
+        np.save(os.path.join(out_dir, "frame_rgba8_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "frame_rgba8.npy"), rgba)
+
+
 class ClockSampler:
     """nvidia-smi clocks / throttle reasons during the timed region (B200_PROFILING.md recipe)."""
 
@@ -67,6 +85,7 @@ class ClockSampler:
         try:
             self.proc = subprocess.Popen(["nvidia-smi", "-i", str(self.index), f"--query-gpu={self.Q}", "--format=csv,noheader,nounits", "-lms", "100"],
                                          stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.stop)  # never outlives the benchmark, even when it fails
             self.t = threading.Thread(target=self._read, daemon=True)
             self.t.start()
         except Exception:
@@ -126,26 +145,32 @@ def ncu_traffic():
 
 # ------------------------------------------------------------------------------------------------
 def _native_oracle():
-    """The oracle rebuilt for THIS machine's cores (-O3 -march=native, BASELINE.md section 4) into
-    oracle/_build/native/: the in-tree liboracle.so is a portable -O2 build because it travels from the
-    build container to the GPU box.  Same sources, same -ffp-contract=off arithmetic contract."""
+    """The oracle rebuilt for THIS machine's cores (-O3 -march=native, BASELINE.md section 4) in a
+    temporary directory (the source tree may be read-only): the in-tree liboracle.so is a portable -O2
+    build because it may be built on another machine.  Same sources, same -ffp-contract=off arithmetic contract."""
+    import shutil
     import subprocess
+    import tempfile
     from oracle import pyoracle as oracle
 
     src_dir = os.path.dirname(os.path.abspath(oracle.__file__))
-    out_dir = os.path.join(src_dir, "_build", "native")
+    in_tree = oracle._LIB_PATH
+    out_dir = tempfile.mkdtemp(prefix="granite_b200_oracle_")
     out = os.path.join(out_dir, "liboracle.so")
     srcs = [os.path.join(src_dir, f) for f in ("oracle_host.c", "oracle_cluster.c", "oracle_lighting.c", "oracle_post.c", "oracle_smaa.c")]
     try:
-        os.makedirs(out_dir, exist_ok=True)
         subprocess.run(["gcc", "-O3", "-march=native", "-std=c11", "-fPIC", "-ffp-contract=off", "-fno-fast-math", "-fopenmp", "-shared", "-o", out,
                         *srcs, "-lm"], check=True, capture_output=True)
         oracle._LIB_PATH = out
         oracle._lib = None
+        oracle.lib()  # loaded now, so the temporary file can go
         return "-O3 -march=native"
     except Exception:
+        oracle._LIB_PATH, oracle._lib = in_tree, None
         oracle.build(ref=False)
         return "-O2 (native rebuild failed)"
+    finally:
+        shutil.rmtree(out_dir, ignore_errors=True)
 
 
 def oracle_frame_time(w, h, n_lights, aa, steps, warmup, budget_s=150.0, bloom=True):
@@ -153,14 +178,14 @@ def oracle_frame_time(w, h, n_lights, aa, steps, warmup, budget_s=150.0, bloom=T
     sample of the frame: the cluster build and the pyramid tail in full, the per-pixel passes on a
     band of rows, scaled to the whole frame.  ONE code path for the `cpu_baseline` key and the
     `--impl reference` arm: native build, threads bound to cores, `warmup` untimed steps, then the
-    MEDIAN of `steps` (>= 3) timed steps."""
+    MEDIAN of `steps` timed steps."""
     os.environ.setdefault("OMP_PROC_BIND", "close")
     os.environ.setdefault("OMP_PLACES", "cores")
     from granite_b200 import synth
     from oracle import pyoracle as oracle
 
     build_flags = _native_oracle()
-    steps = max(int(steps), 3)
+    steps = max(int(steps), 1)
     warmup = max(int(warmup), 1)
     cores = os.cpu_count() or 1
     scene = synth.make_scene(w, h)
@@ -235,7 +260,11 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="c3", choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the output frame of the last timed step to DIR/*.npy (all ranks' rows, written by rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     w, h, n_lights, aa, desc = WORKLOADS[args.workload]
@@ -254,7 +283,9 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return 0
-        steps = max(min(args.steps, 200), 3)  # the row sample inside oracle_frame_time bounds the run to a few minutes
+        # the row sample inside oracle_frame_time fits the run into its budget down to a band of 64 rows per step;
+        # beyond that the run time grows with --steps
+        steps = args.steps
         sec, cores, sample = oracle_frame_time(w, h, n_lights, aa, steps, 1, bloom=bloom)
         fps = 1.0 / sec
         line = {"impl": "reference", "metric": "frames/sec", "value": fps, "unit": "frames/s", "n_gpus": args.gpus, "steps": steps,
@@ -382,21 +413,21 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item())
 
-    # warm-up: uploads the G-buffer, builds the history images, adapts the luminance
-    for _ in range(args.warmup):
-        v.render_frame(gb)
-        v.read_output(out)
-
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
         time.sleep(0.3)
 
+    # warm-up: uploads the G-buffer, builds the history images, adapts the luminance.  It runs after the
+    # sampler's start-up pause, so that the single timed window follows a busy device, not an idle one.
+    for _ in range(args.warmup):
+        v.render_frame(gb)
+        v.read_output(out)
+
     # ---- timed region 1: device-resident inputs (value) ----
-    # A window is EXACTLY K steps between two events (barrier + synchronize on both sides, max over
-    # ranks).  K frames of this workload last a few milliseconds, which is too short to be a steady
-    # state on its own, so the window is repeated until at least 0.5 s of GPU time has been timed and
-    # `value` is the MEDIAN window (all windows are reported).
+    # ONE window of EXACTLY K steps between two events (barrier + synchronize on both sides, max over
+    # ranks).  A frame of c3 lasts about half a millisecond on a B200, so a window long enough to be
+    # a steady state wants K of a few hundred (the default, 200, times about 0.1 s).
     PREROLL = 4
 
     def resident_window():
@@ -419,16 +450,26 @@ def main():
         return max_over_ranks(e0.elapsed_time(e1)), host
 
     t_begin = time.time()
-    windows, hosts = [], []
-    while not windows or (sum(windows) < 500.0 and len(windows) < 400):
-        ms, host = resident_window()
-        windows.append(ms)
-        hosts.append(host)
-    ms_resident = float(np.median(windows))
-    host_ms = float(np.median(hosts))
-    srt = sorted(windows)
-    frame_stats = {"windows": len(windows), "steps_per_window": args.steps, "preroll_frames": PREROLL, "min": round(srt[0] / args.steps, 4), "p50": round(ms_resident / args.steps, 4),
-                   "max": round(srt[-1] / args.steps, 4)}
+    ms_resident, host_ms = resident_window()
+    frame_stats = {"windows": 1, "steps_per_window": args.steps, "preroll_frames": PREROLL}
+    if args.dump_outputs:
+        y0, y1 = v.read_output(out)  # the frame of the last timed step, as a caller of the viewer receives it
+        frame = out.numpy()
+        if world > 1:  # each rank holds its band of rows: rank 0 assembles the whole frame
+            parts = [torch.zeros((h, w), dtype=torch.int32, device="cuda") for _ in range(world)]
+            spans = [torch.zeros(2, dtype=torch.int64, device="cuda") for _ in range(world)]
+            dist.all_gather(parts, out.cuda())
+            dist.all_gather(spans, torch.tensor([y0, y1], dtype=torch.int64, device="cuda"))
+            frame = np.zeros((h, w), np.int32)
+            covered = np.zeros(h, bool)
+            for part, span in zip(parts, spans):
+                a, b = (int(x) for x in span.tolist())
+                frame[a:b] = part[a:b].cpu().numpy()
+                covered[a:b] = True
+            assert covered.all(), "the ranks' output bands do not cover the frame"
+            y0, y1 = 0, h
+        if rank == 0:
+            dump_outputs(args.dump_outputs, frame[y0:y1])
 
     # ---- timed region 2: end to end through the host API.  Every step copies its G-buffer rows from
     # pinned host memory to the device and its result rows back; frames are pipelined two deep (the

@@ -49,7 +49,7 @@ static int32_t poll_device_error(const char *what)
 	const uint32_t code = *w;
 	*w = 0u; // reported once
 	if ((code >> 24) == GRB_DEVICE_ERROR_PEER_TIMEOUT)
-		std::snprintf(t_last_error, sizeof(t_last_error), "%s: an earlier wait for the peers' bands (grb_peer_wait / grb_bloom_tail_ex) timed out on rank %u's band (frame epoch %u, low 16 bits); the "
+		std::snprintf(t_last_error, sizeof(t_last_error), "%s: an earlier wait for the peers' bands (grb_peer_wait / grb_bloom_tail_ex) timed out waiting for rank %u's band (frame epoch %u, low 16 bits); the "
 		              "frame that followed used stale data", what, (code >> 16) & 0xffu, code & 0xffffu);
 	else
 		std::snprintf(t_last_error, sizeof(t_last_error), "%s: device-side error word 0x%08x", what, code);

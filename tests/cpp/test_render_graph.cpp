@@ -49,7 +49,7 @@ static std::string join(const std::vector<std::string> &v)
 	return s;
 }
 
-int main()
+int main(int argc, char **argv)
 {
 	ResourceDimensions dim;
 	dim.width = 3840;
@@ -392,10 +392,12 @@ int main()
 		CHECK(!parse_gtx(file.data(), 63, img, err) && !parse_gtx(file.data(), file.size() - 1, img, err));
 		file[0] = 'X';
 		CHECK(!parse_gtx(file.data(), file.size(), img, err));
-		// the reference's own files, where they exist
-		GtxImage area, search;
-		if (load_gtx("/root/reference/assets/textures/smaa/area.gtx", area, err) && load_gtx("/root/reference/assets/textures/smaa/search.gtx", search, err))
+		// the reference's SMAA lookup textures, from the directory given as the first argument
+		if (argc > 1)
 		{
+			const std::string dir = argv[1];
+			GtxImage area, search;
+			CHECK(load_gtx(dir + "/area.gtx", area, err) && load_gtx(dir + "/search.gtx", search, err));
 			CHECK(area.format == VK_FORMAT_R8G8_UNORM && area.width == 160 && area.height == 560 && area.texels.size() == 160u * 560u * 2u);
 			CHECK(search.format == VK_FORMAT_R8_UNORM && search.width == 64 && search.height == 16 && search.texels.size() == 1024u);
 		}

@@ -87,15 +87,34 @@ def test_product_sources_never_touch_the_oracle():
     assert not bad, f"product files reference the oracle: {bad}"
 
 
+def _smaa_lut_dir(tmp_path):
+    """The reference's SMAA lookup textures: its own asset directory where it exists, else the same texels (recorded
+    from those files in tests/golden/refsmaa_160x96.npz) in .gtx containers written to tmp_path."""
+    from oracle import pyoracle
+
+    if os.path.isdir(pyoracle.SMAA_LUT_DIR):
+        return pyoracle.SMAA_LUT_DIR
+    f = np.load(os.path.join(ROOT, "tests", "golden", "refsmaa_160x96.npz"))
+    for name, fmt in (("area", 16), ("search", 9)):  # VK_FORMAT_R8G8_UNORM, VK_FORMAT_R8_UNORM
+        texels = np.ascontiguousarray(f[name])
+        h, w, _ = texels.shape
+        # 64-byte header (memory_mapped_texture.cpp:29-46): magic, 2-D type, format, size, depth, layers, levels, flags, payload
+        header = b"GRANITE TEXFMT1\0" + np.array([1, fmt, w, h, 1, 1, 1, 0], np.uint32).tobytes() + np.uint64(texels.size).tobytes() + bytes(8)
+        (tmp_path / f"{name}.gtx").write_bytes(header + texels.tobytes())
+    return str(tmp_path)
+
+
 def test_render_graph_cpp(built, tmp_path):
     exe = str(tmp_path / "test_render_graph")
+    luts = tmp_path / "smaa"
+    luts.mkdir()
     cuda = os.environ.get("CUDA_HOME", "/usr/local/cuda")
     libdir = os.path.join(ROOT, "granite_b200")
     cmd = ["g++", "-O1", "-std=c++17", f"-I{cuda}/include", os.path.join(ROOT, "tests", "cpp", "test_render_graph.cpp"), "-o", exe,
            f"-L{libdir}", "-lgranite_b200_host", "-lgranite_b200", f"-Wl,-rpath,{libdir}", f"-Wl,-rpath,{cuda}/lib64"]
     r = subprocess.run(cmd, capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
-    r = subprocess.run([exe], capture_output=True, text=True)
+    r = subprocess.run([exe, _smaa_lut_dir(luts)], capture_output=True, text=True)
     assert r.returncode == 0, r.stdout + r.stderr
 
 
@@ -169,16 +188,18 @@ def test_hdr10_output_rejects_fxaa(built):
     v.close()
 
 
-def test_gtx_reader_reads_the_reference_lookup_textures(built, oracle):
-    """The host library's .gtx reader (host/post/smaa.cpp) against the Python reader the oracle tests use."""
+def test_gtx_reader_reads_the_reference_lookup_textures(built, oracle, tmp_path):
+    """The host library's .gtx reader (host/post/smaa.cpp) against the Python reader the oracle tests use, on the
+    reference's lookup textures, whose texels the SMAA fixture holds."""
     from granite_b200 import capi, viewer
 
-    if not os.path.isdir(oracle.SMAA_LUT_DIR):
-        pytest.skip("the reference's assets are not on this machine")
-    area, search = oracle.smaa_luts()
-    fmt, a = viewer.load_gtx(os.path.join(oracle.SMAA_LUT_DIR, "area.gtx"))
+    d = _smaa_lut_dir(tmp_path)
+    area, search = oracle.load_gtx(os.path.join(d, "area.gtx")), oracle.load_gtx(os.path.join(d, "search.gtx"))
+    f = np.load(os.path.join(ROOT, "tests", "golden", "refsmaa_160x96.npz"))
+    assert np.array_equal(area, f["area"]) and np.array_equal(search, f["search"])
+    fmt, a = viewer.load_gtx(os.path.join(d, "area.gtx"))
     assert fmt == capi.FORMAT_R8G8_UNORM and np.array_equal(a, area)
-    fmt, s = viewer.load_gtx(os.path.join(oracle.SMAA_LUT_DIR, "search.gtx"))
+    fmt, s = viewer.load_gtx(os.path.join(d, "search.gtx"))
     assert fmt == capi.FORMAT_R8_UNORM and np.array_equal(s, search)
     with pytest.raises(RuntimeError):
         viewer.load_gtx("/nonexistent.gtx")
