@@ -14,6 +14,7 @@
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>
+#include <type_traits>
 
 namespace grb
 {
@@ -616,14 +617,37 @@ struct Mat4
 	float m[16];
 };
 
-template <int Quality, bool History, typename HdrTexel = uint32_t>
-__global__ void __launch_bounds__(kBlockX *kBlockY) taa_kernel(TaaInputsT<HdrTexel> in, Mat4 reproj, View<uint32_t> out_color, View<uint2> out_history, int y0,
-                                                              int y1, float4 rt)
+// The history exchange of a row-sharded frame (the peer form of the resolve): the history texels of the rows
+// [own_y0, own_y1) go to the history slot of every rank instead of out_history, then the last CTA raises
+// flags[flag_index] = epoch on every rank (as bloom_downsample_peers_kernel).  NoTaaPeerStore: the plain resolve.
+struct NoTaaPeerStore
 {
+};
+struct TaaPeerStore
+{
+	PeerTargets targets;
+	int pitch_texels, own_y0, own_y1, flag_index;
+	uint32_t epoch;
+	unsigned *ctas_done;
+};
+
+template <int Quality, bool History, typename HdrTexel = uint32_t, typename PeerStore = NoTaaPeerStore>
+__global__ void __launch_bounds__(kBlockX *kBlockY) taa_kernel(TaaInputsT<HdrTexel> in, Mat4 reproj, View<uint32_t> out_color, View<uint2> out_history, int y0,
+                                                              int y1, float4 rt, PeerStore peers)
+{
+	constexpr bool kPeers = std::is_same<PeerStore, TaaPeerStore>::value;
 	int x = blockIdx.x * kBlockX + threadIdx.x;
 	int y = y0 + blockIdx.y * kBlockY + threadIdx.y;
-	if (x >= out_color.w || y >= y1)
-		return;
+	const bool inside = x < out_color.w && y < y1;
+	if (!inside)
+	{
+		if (!kPeers)
+			return;
+		// every thread of the peer form reaches the CTA barrier of the epilogue: off the image it resolves a clamped
+		// pixel and stores nothing
+		x = min(x, out_color.w - 1);
+		y = min(y, y1 - 1);
+	}
 	const int w = in.hdr.w, h = in.hdr.h;
 #define GRB_CUR(DX, DY) hdr_to_taa(fetch_hdr_clamped(in.hdr, x + (DX), y + (DY)))
 	float3 current = GRB_CUR(0, 0);
@@ -727,8 +751,41 @@ __global__ void __launch_bounds__(kBlockX *kBlockY) taa_kernel(TaaInputsT<HdrTex
 	}
 #undef GRB_CUR
 	float3 color = taa_to_hdr(out_c);
-	out_color.at(x, y) = pack_r11g11b10(color.x, color.y, color.z);
-	out_history.at(x, y) = pack_rgba16f(make_float4(out_c.x, out_c.y, out_c.z, 1.0f));
+	if constexpr (!kPeers)
+	{
+		out_color.at(x, y) = pack_r11g11b10(color.x, color.y, color.z);
+		out_history.at(x, y) = pack_rgba16f(make_float4(out_c.x, out_c.y, out_c.z, 1.0f));
+	}
+	else
+	{
+		if (inside)
+		{
+			out_color.at(x, y) = pack_r11g11b10(color.x, color.y, color.z);
+			if (y >= peers.own_y0 && y < peers.own_y1)
+			{
+				const uint2 texel = pack_rgba16f(make_float4(out_c.x, out_c.y, out_c.z, 1.0f));
+				const size_t at = (size_t)y * peers.pitch_texels + x;
+				for (int r = 0; r < peers.targets.count; r++)
+					peers.targets.data[r][at] = texel;
+			}
+		}
+		// publish (threadFenceReduction pattern at system scope, as bloom_downsample_peers_kernel): every CTA has read
+		// its history texels and stored its band texels before it arrives, so a raised flag also says "this rank is
+		// done reading last frame's slot"
+		__threadfence_system();
+		__syncthreads();
+		if (threadIdx.x == 0 && threadIdx.y == 0)
+		{
+			const unsigned total = gridDim.x * gridDim.y;
+			if (atomicAdd(peers.ctas_done, 1u) == total - 1u)
+			{
+				*peers.ctas_done = 0u;
+				__threadfence_system();
+				for (int r = 0; r < peers.targets.count; r++)
+					store_release_system(peers.targets.flags[r] + peers.flag_index, peers.epoch);
+			}
+		}
+	}
 }
 
 // ------------------------------------------------------------------------------- pyramid tail
@@ -1189,15 +1246,20 @@ extern "C" int32_t grb_fxaa(const GrbImage *in, const GrbImage *out, GrbRows row
 	return check_launch("grb_fxaa");
 }
 
-extern "C" int32_t grb_taa_resolve(const GrbImage *hdr, const GrbImage *depth, const GrbImage *mv, const GrbImage *history, const float *reproj16,
-                                   int32_t quality, const GrbImage *out_color, const GrbImage *out_history, GrbRows rows, void *stream)
+// Argument checks shared by grb_taa_resolve and grb_taa_resolve_to_peers (`what` names the entry point).  The
+// history image the call writes is out_history (its layout only, for the peer form); with history it must not be the
+// image the call reads.
+static int32_t taa_arguments_ok(const char *what, const GrbImage *hdr, const GrbImage *depth, const GrbImage *mv, const GrbImage *history,
+                                const float *reproj16, int32_t quality, const GrbImage *out_color, const GrbImage *out_history, bool *hdr16_out)
 {
+	char msg[256];
 	const bool hdr16 = image_ok(hdr, GRB_FORMAT_R16G16B16A16_SFLOAT, 8); // "renderTargetFp16": the resolve's own output stays B10G11R11 (temporal.cpp:209-212)
 	if ((!hdr16 && !image_ok(hdr, GRB_FORMAT_B10G11R11_UFLOAT_PACK32, 4)) || !image_ok(out_color, GRB_FORMAT_B10G11R11_UFLOAT_PACK32, 4) ||
 	    !image_ok(out_history, GRB_FORMAT_R16G16B16A16_SFLOAT, 8) || out_color->width != hdr->width || out_color->height != hdr->height ||
 	    out_history->width != hdr->width || out_history->height != hdr->height)
 	{
-		set_last_error("grb_taa_resolve: hdr B10G11R11_UFLOAT or R16G16B16A16_SFLOAT, out_color B10G11R11_UFLOAT, out_history R16G16B16A16_SFLOAT, equal sizes");
+		snprintf(msg, sizeof(msg), "%s: hdr B10G11R11_UFLOAT or R16G16B16A16_SFLOAT, out_color B10G11R11_UFLOAT, out_history R16G16B16A16_SFLOAT, equal sizes", what);
+		set_last_error(msg);
 		return GRB_ERR_UNSUPPORTED_FORMAT;
 	}
 	if (history && (!image_ok(history, GRB_FORMAT_R16G16B16A16_SFLOAT, 8) || !image_ok(depth, GRB_FORMAT_D32_SFLOAT, 4) ||
@@ -1205,23 +1267,26 @@ extern "C" int32_t grb_taa_resolve(const GrbImage *hdr, const GrbImage *depth, c
 	                depth->width != hdr->width || depth->height != hdr->height || mv->width != hdr->width || mv->height != hdr->height ||
 	                history->data == out_history->data))
 	{
-		set_last_error("grb_taa_resolve: with history, depth (D32_SFLOAT), mv (R16G16_SFLOAT), reproj and a distinct history image are required");
+		snprintf(msg, sizeof(msg), "%s: with history, depth (D32_SFLOAT), mv (R16G16_SFLOAT), reproj and a distinct history image are required", what);
+		set_last_error(msg);
 		return GRB_ERR_INVALID_ARGUMENT;
 	}
 	if (quality < 0 || quality > 2)
 	{
-		set_last_error("grb_taa_resolve: quality must be 0..2");
+		snprintf(msg, sizeof(msg), "%s: quality must be 0..2", what);
+		set_last_error(msg);
 		return GRB_ERR_INVALID_ARGUMENT;
 	}
-	rows = full_rows(rows, hdr->height);
-	if (rows.y1 <= rows.y0)
-		return GRB_OK;
-	if (history && quality == 2 && !hdr16)
-	{
-		int32_t rc = GRB_OK;
-		if (launch_taa_fast(hdr, depth, mv, history, reproj16, out_color, out_history, rows, as_stream(stream), &rc))
-			return rc;
-	}
+	*hdr16_out = hdr16;
+	return GRB_OK;
+}
+
+// The exact resolve (taa_kernel) over `rows`, for both HDR texel types, all qualities, with and without history;
+// PeerStore selects the plain form (out_history) or the peer form (TaaPeerStore).
+template <typename PeerStore>
+static void launch_taa_exact(bool hdr16, const GrbImage *hdr, const GrbImage *depth, const GrbImage *mv, const GrbImage *history, const float *reproj16,
+                             int32_t quality, const GrbImage *out_color, View<uint2> oh, GrbRows rows, cudaStream_t s, const PeerStore &peers)
+{
 	TaaInputs in{};
 	in.hdr = view_of<const uint32_t>(hdr);
 	Mat4 m{};
@@ -1234,10 +1299,8 @@ extern "C" int32_t grb_taa_resolve(const GrbImage *hdr, const GrbImage *depth, c
 			m.m[i] = reproj16[i];
 	}
 	auto oc = view_of<uint32_t>(out_color);
-	auto oh = view_of<uint2>(out_history);
 	float4 rt = make_float4(1.0f / (float)hdr->width, 1.0f / (float)hdr->height, (float)hdr->width, (float)hdr->height); // temporal.cpp:245-248
 	dim3 grid = grid_for(hdr->width, rows.y1 - rows.y0), block(kBlockX, kBlockY);
-	cudaStream_t s = as_stream(stream);
 	if (hdr16)
 	{
 		TaaInputsT<uint2> in16{};
@@ -1245,7 +1308,7 @@ extern "C" int32_t grb_taa_resolve(const GrbImage *hdr, const GrbImage *depth, c
 		in16.depth = in.depth;
 		in16.mv = in.mv;
 		in16.history = in.history;
-#define GRB_LAUNCH16(Q, H) taa_kernel<Q, H, uint2><<<grid, block, 0, s>>>(in16, m, oc, oh, rows.y0, rows.y1, rt)
+#define GRB_LAUNCH16(Q, H) taa_kernel<Q, H, uint2, PeerStore><<<grid, block, 0, s>>>(in16, m, oc, oh, rows.y0, rows.y1, rt, peers)
 		if (!history)
 			GRB_LAUNCH16(0, false);
 		else if (quality == 0)
@@ -1255,9 +1318,9 @@ extern "C" int32_t grb_taa_resolve(const GrbImage *hdr, const GrbImage *depth, c
 		else
 			GRB_LAUNCH16(2, true);
 #undef GRB_LAUNCH16
-		return check_launch("grb_taa_resolve");
+		return;
 	}
-#define GRB_LAUNCH(Q, H) taa_kernel<Q, H><<<grid, block, 0, s>>>(in, m, oc, oh, rows.y0, rows.y1, rt)
+#define GRB_LAUNCH(Q, H) taa_kernel<Q, H, uint32_t, PeerStore><<<grid, block, 0, s>>>(in, m, oc, oh, rows.y0, rows.y1, rt, peers)
 	if (!history)
 		GRB_LAUNCH(0, false);
 	else if (quality == 0)
@@ -1267,7 +1330,79 @@ extern "C" int32_t grb_taa_resolve(const GrbImage *hdr, const GrbImage *depth, c
 	else
 		GRB_LAUNCH(2, true);
 #undef GRB_LAUNCH
+}
+
+extern "C" int32_t grb_taa_resolve(const GrbImage *hdr, const GrbImage *depth, const GrbImage *mv, const GrbImage *history, const float *reproj16,
+                                   int32_t quality, const GrbImage *out_color, const GrbImage *out_history, GrbRows rows, void *stream)
+{
+	bool hdr16 = false;
+	if (int32_t rc = taa_arguments_ok("grb_taa_resolve", hdr, depth, mv, history, reproj16, quality, out_color, out_history, &hdr16))
+		return rc;
+	rows = full_rows(rows, hdr->height);
+	if (rows.y1 <= rows.y0)
+		return GRB_OK;
+	if (history && quality == 2 && !hdr16)
+	{
+		int32_t rc = GRB_OK;
+		if (launch_taa_fast(hdr, depth, mv, history, reproj16, out_color, out_history, rows, as_stream(stream), &rc))
+			return rc;
+	}
+	launch_taa_exact(hdr16, hdr, depth, mv, history, reproj16, quality, out_color, view_of<uint2>(out_history), rows, as_stream(stream), NoTaaPeerStore{});
 	return check_launch("grb_taa_resolve");
+}
+
+extern "C" int32_t grb_taa_resolve_to_peers(const GrbImage *hdr, const GrbImage *depth, const GrbImage *mv, const GrbImage *history, const float *reproj16,
+                                            int32_t quality, const GrbImage *out_color, const GrbImage *out_history_layout, void *const *peer_images,
+                                            uint32_t *const *peer_flags, int32_t peer_count, int32_t flag_index, uint32_t epoch,
+                                            uint32_t *scratch_counter, GrbRows rows, GrbRows own_rows, void *stream)
+{
+	if (!hdr || !out_history_layout || !peer_images || !peer_flags || !scratch_counter || peer_count < 1 || peer_count > GRB_MAX_PEERS ||
+	    flag_index < 0 || flag_index >= peer_count)
+	{
+		set_last_error("grb_taa_resolve_to_peers: bad arguments (out_history_layout, peer_images, peer_flags, scratch_counter; peer_count 1..GRB_MAX_PEERS, "
+		               "0 <= flag_index < peer_count)");
+		return GRB_ERR_INVALID_ARGUMENT;
+	}
+	for (int r = 0; r < peer_count; r++)
+		if (!peer_images[r] || !peer_flags[r])
+		{
+			set_last_error("grb_taa_resolve_to_peers: null peer pointer");
+			return GRB_ERR_INVALID_ARGUMENT;
+		}
+	// the layout describes every rank's history slot; its data pointer is not written (only the peer images are)
+	GrbImage layout = *out_history_layout;
+	if (!layout.data)
+		layout.data = peer_images[0];
+	bool hdr16 = false;
+	if (int32_t rc = taa_arguments_ok("grb_taa_resolve_to_peers", hdr, depth, mv, history, reproj16, quality, out_color, &layout, &hdr16))
+		return rc;
+	TaaPeerStore peers{};
+	peers.targets.count = peer_count;
+	for (int r = 0; r < peer_count; r++)
+	{
+		if (history && history->data == peer_images[r])
+		{
+			set_last_error("grb_taa_resolve_to_peers: the history image read must not be a history slot this call writes");
+			return GRB_ERR_INVALID_ARGUMENT;
+		}
+		peers.targets.data[r] = static_cast<uint2 *>(peer_images[r]);
+		peers.targets.flags[r] = peer_flags[r];
+	}
+	rows = full_rows(rows, hdr->height);
+	own_rows = full_rows(own_rows, hdr->height);
+	if (rows.y1 <= rows.y0 || own_rows.y1 <= own_rows.y0 || own_rows.y0 < rows.y0 || own_rows.y1 > rows.y1)
+	{
+		set_last_error("grb_taa_resolve_to_peers: rows and own_rows must be non-empty, own_rows inside rows");
+		return GRB_ERR_INVALID_ARGUMENT;
+	}
+	peers.pitch_texels = layout.row_pitch / 8;
+	peers.own_y0 = own_rows.y0;
+	peers.own_y1 = own_rows.y1;
+	peers.flag_index = flag_index;
+	peers.epoch = epoch;
+	peers.ctas_done = scratch_counter;
+	launch_taa_exact(hdr16, hdr, depth, mv, history, reproj16, quality, out_color, View<uint2>{}, rows, as_stream(stream), peers);
+	return check_launch("grb_taa_resolve_to_peers");
 }
 
 // d1 .. d3 (+ temporal feedback), the average-luminance update, u2 and u1 in one cooperative launch

@@ -86,7 +86,8 @@ bool nccl_ok(int rc, const char *what)
 
 NcclCollectives::~NcclCollectives()
 {
-	release_peer_exchange();
+	release_peer_exchange(peer);
+	release_peer_exchange(taa_history);
 	if (comm && api().CommDestroy)
 		api().CommDestroy(comm);
 }
@@ -177,7 +178,7 @@ bool NcclCollectives::all_reduce_sum(Vulkan::CommandBuffer &cmd, float *data, si
 }
 
 // ----------------------------------------------------------------------------- peer exchange
-void NcclCollectives::release_peer_exchange()
+void NcclCollectives::release_peer_exchange(PeerState &peer)
 {
 	for (void *p : peer.opened)
 		cudaIpcCloseMemHandle(p);
@@ -194,7 +195,7 @@ void NcclCollectives::release_peer_exchange()
 	peer.ok = false;
 }
 
-bool NcclCollectives::setup_peer_exchange(size_t image_bytes)
+bool NcclCollectives::setup_peer_exchange(PeerState &peer, size_t image_bytes)
 {
 	// Collective: every rank calls this with the same size at the same point of its first sharded frame.
 	struct Handles
@@ -264,25 +265,27 @@ bool NcclCollectives::setup_peer_exchange(size_t image_bytes)
 		cudaGetLastError();
 		if (!(mode && std::string(mode) == "nccl"))
 			Vulkan::log_info("peer-memory exchange unavailable on rank %u (no IPC / peer access); using NCCL broadcasts.\n", rank);
-		release_peer_exchange();
+		release_peer_exchange(peer);
 		return false;
 	}
 	peer.image_bytes = image_bytes;
+	peer.frames = 0;
 	return true;
 }
 
-bool NcclCollectives::peer_exchange_begin_frame(size_t image_bytes, PeerSlot &slot)
+bool NcclCollectives::begin_frame(PeerState &peer, size_t image_bytes, PeerSlot &slot)
 {
 	if (!peer.tried || (peer.ok && peer.image_bytes != image_bytes))
 	{
 		// (a re-bake at another size re-creates the buffers; all ranks re-bake together)
 		if (peer.tried)
-			release_peer_exchange();
+			release_peer_exchange(peer);
 		peer.tried = true;
-		peer.ok = setup_peer_exchange(image_bytes);
+		peer.ok = setup_peer_exchange(peer, image_bytes);
 	}
 	if (!peer.ok)
 		return false;
+	peer.frames++;
 	peer.epoch++;
 	const unsigned k = peer.epoch & 1u;
 	slot.count = world;
@@ -293,6 +296,21 @@ bool NcclCollectives::peer_exchange_begin_frame(size_t image_bytes, PeerSlot &sl
 		slot.images[r] = peer.images[k][r];
 		slot.flags[r] = peer.flags[r];
 	}
+	return true;
+}
+
+bool NcclCollectives::peer_exchange_begin_frame(size_t image_bytes, PeerSlot &slot)
+{
+	return begin_frame(peer, image_bytes, slot);
+}
+
+bool NcclCollectives::taa_history_begin_frame(size_t image_bytes, PeerSlot &slot, void *&previous)
+{
+	previous = nullptr;
+	if (!begin_frame(taa_history, image_bytes, slot))
+		return false;
+	if (taa_history.frames > 1)
+		previous = taa_history.local_images[(taa_history.epoch - 1) & 1u];
 	return true;
 }
 } // namespace Granite

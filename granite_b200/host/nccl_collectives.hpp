@@ -28,6 +28,8 @@ public:
 	// Peer-memory exchange: two image slots + a flag array per rank, cudaIpc-mapped into every
 	// other rank (handles are exchanged with one ncclAllGather).  GRB_SHARD_EXCHANGE=nccl disables it.
 	bool peer_exchange_begin_frame(size_t image_bytes, PeerSlot &slot) override;
+	// The TAA history channel: a second set of the same buffers.
+	bool taa_history_begin_frame(size_t image_bytes, PeerSlot &slot, void *&previous) override;
 
 private:
 	bool collective_failed(const char *what);
@@ -44,8 +46,10 @@ private:
 		uint32_t *flags[8] = {};
 		std::vector<void *> opened;
 		uint32_t epoch = 0;
-	} peer;
-	bool setup_peer_exchange(size_t image_bytes);
-	void release_peer_exchange();
+		unsigned frames = 0; // frames begun since the buffers were (re-)created
+	} peer, taa_history;
+	bool begin_frame(PeerState &peer, size_t image_bytes, PeerSlot &slot);
+	bool setup_peer_exchange(PeerState &peer, size_t image_bytes);
+	void release_peer_exchange(PeerState &peer);
 };
 } // namespace Granite

@@ -120,11 +120,6 @@ void setup_taa_resolve(RenderGraph &graph, TemporalJitter &jitter, float scaling
 
 	resolve.set_build_render_pass([&graph, &jitter, &out_color, &out_history, &input_res, &input_res_mv, &input_depth_res, &history,
 	                               q = int(quality)](Vulkan::CommandBuffer &cmd) {
-		if (graph.is_sharded() && graph.get_shard_count() > 1)
-		{
-			Vulkan::log_error("taa-resolve: row-sharded frames are not supported (history rows would need a halo exchange).\n");
-			return;
-		}
 		GrbImage image = graph.get_physical_texture_resource(input_res).as_grb();
 		GrbImage image_mv = graph.get_physical_texture_resource(input_res_mv).as_grb();
 		GrbImage depth = graph.get_physical_texture_resource(input_depth_res).as_grb();
@@ -138,6 +133,43 @@ void setup_taa_resolve(RenderGraph &graph, TemporalJitter &jitter, float scaling
 		// temporal.cpp:239-243: clip(now) -> UV(previous frame)
 		mat4 reproj = translate(vec3(0.5f, 0.5f, 0.0f)) * scale(vec3(0.5f, 0.5f, 1.0f)) * jitter.get_history_view_proj(1) *
 		              jitter.get_history_inv_view_proj(0);
+		if (graph.is_sharded() && graph.get_shard_count() > 1)
+		{
+			// Row-sharded frames: a pixel reads last frame's history at its reprojected position, which can be anywhere
+			// in the frame, so every rank holds the whole history.  This rank resolves plan.taa (what the threshold and
+			// the tonemap read) and contributes the history of its own band.
+			const ShardPlan plan = graph.get_shard_plan();
+			auto *collectives = graph.get_collectives();
+			const unsigned self = collectives->get_rank();
+			RenderGraphCollectives::PeerSlot slot;
+			void *previous = nullptr;
+			if (collectives->taa_history_begin_frame((size_t)oh.row_pitch * (size_t)oh.height, slot, previous))
+			{
+				// Peer path: the resolve stores its band into this frame's slot on every rank, the previous frame's slot
+				// is the history.  Two slots suffice: before its frame N+1 resolve a rank waits until every rank's
+				// frame-N flag has arrived (it needs that wait anyway to read the history), and a rank raises that flag
+				// at the end of its frame-N resolve, after reading slot (N-1) mod 2.  So by the time a rank stores into
+				// slot (N+1) mod 2 on a peer, that peer has finished reading it.  The wait is kept on the first frame
+				// after a re-bake too (no history is read then, but the slot is still reused).
+				if (previous)
+					cmd.check(grb_peer_wait(slot.flags[self], (int32_t)slot.count, slot.epoch - 1u, cmd.get_stream_handle()), "grb_peer_wait(taa history)");
+				GrbImage full_history = oh;
+				full_history.data = previous;
+				cmd.check(grb_taa_resolve_to_peers(&image, &depth, &image_mv, prev && previous ? &full_history : nullptr, reproj.data(), q, &oc, &oh,
+				                                   slot.images, slot.flags, (int32_t)slot.count, (int32_t)self, slot.epoch, slot.counter, plan.taa,
+				                                   plan.own, cmd.get_stream_handle()),
+				          "grb_taa_resolve_to_peers");
+				return;
+			}
+			// NCCL path: resolve into the graph's history image, then every rank broadcasts its band of it
+			cmd.check(grb_taa_resolve(&image, &depth, &image_mv, prev ? &prev_img : nullptr, reproj.data(), q, &oc, &oh, plan.taa, cmd.get_stream_handle()),
+			          "grb_taa_resolve");
+			std::vector<GrbRows> bands;
+			for (unsigned rank = 0; rank < graph.get_shard_count(); rank++)
+				bands.push_back(graph.get_shard_plan(rank).own);
+			collectives->all_gather_rows(cmd, graph.get_physical_texture_resource(out_history), bands);
+			return;
+		}
 		cmd.check(grb_taa_resolve(&image, &depth, &image_mv, prev ? &prev_img : nullptr, reproj.data(), q, &oc, &oh, GrbRows{ 0, 0 },
 		                          cmd.get_stream_handle()),
 		          "grb_taa_resolve");

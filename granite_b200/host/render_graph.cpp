@@ -774,9 +774,11 @@ void RenderGraph::log()
 	}
 }
 
-void RenderGraph::set_row_shards(const std::vector<GrbRows> &bands, unsigned rank, RenderGraphCollectives *collectives_, bool fxaa_downstream)
+void RenderGraph::set_row_shards(const std::vector<GrbRows> &bands, unsigned rank, RenderGraphCollectives *collectives_, bool fxaa_downstream,
+                                 bool taa_upstream)
 {
 	shard_fxaa = fxaa_downstream;
+	shard_taa = taa_upstream;
 	if (!bands.empty())
 	{
 		if (rank >= bands.size())

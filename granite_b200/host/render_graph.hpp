@@ -70,6 +70,17 @@ public:
 		(void)slot;
 		return false;
 	}
+	// The same kind of exchange for the TAA history, as a channel of its own (its own double-buffered image, flag
+	// arrays and scratch counter: the resolve runs on another stream than the bloom exchange).  Besides this frame's
+	// slot it returns `previous`, this rank's copy of the previous frame's slot: the full history the resolve reads
+	// (nullptr on the channel's first frame).  false = not available: callers then use all_gather_rows().
+	virtual bool taa_history_begin_frame(size_t image_bytes, PeerSlot &slot, void *&previous)
+	{
+		(void)image_bytes;
+		(void)slot;
+		previous = nullptr;
+		return false;
+	}
 };
 
 class RenderPassInterface
@@ -461,12 +472,13 @@ public:
 	// Row-sharded frames (multi-GPU, one graph per device/process): `bands[r]` = backbuffer rows
 	// [y0, y1) owned by rank r; they must tile the frame.  Builders scale the local band per
 	// resource with shard_rows_for(); an unsharded graph returns {0,0} (= all rows).
-	void set_row_shards(const std::vector<GrbRows> &bands, unsigned rank, RenderGraphCollectives *collectives, bool fxaa_downstream = false);
+	void set_row_shards(const std::vector<GrbRows> &bands, unsigned rank, RenderGraphCollectives *collectives, bool fxaa_downstream = false,
+	                    bool taa_upstream = false);
 	// Rows of every stage for `rank` (this rank by default); whole images when unsharded.
 	ShardPlan get_shard_plan() const { return get_shard_plan(shard_rank); }
 	ShardPlan get_shard_plan(unsigned rank) const
 	{
-		return compute_shard_plan(swapchain_dimensions.width, swapchain_dimensions.height, shard_bands, rank, shard_fxaa);
+		return compute_shard_plan(swapchain_dimensions.width, swapchain_dimensions.height, shard_bands, rank, shard_fxaa, shard_taa);
 	}
 	GrbRows shard_rows_for(unsigned resource_height, unsigned halo_rows = 0) const;
 	GrbRows shard_rows_for_rank(unsigned rank, unsigned resource_height, unsigned halo_rows = 0) const;
@@ -527,6 +539,7 @@ private:
 	std::vector<GrbRows> shard_bands;
 	unsigned shard_rank = 0;
 	bool shard_fxaa = false;
+	bool shard_taa = false;
 	RenderGraphCollectives *collectives = nullptr;
 
 	RenderTextureResource &get_or_create_texture(const std::string &name);

@@ -28,7 +28,7 @@ GrbRows scale_band(GrbRows band, unsigned from_h, unsigned to_h)
 }
 } // namespace
 
-ShardPlan compute_shard_plan(unsigned, unsigned height, const std::vector<GrbRows> &bands, unsigned rank, bool fxaa)
+ShardPlan compute_shard_plan(unsigned, unsigned height, const std::vector<GrbRows> &bands, unsigned rank, bool fxaa, bool taa)
 {
 	ShardPlan p = {};
 	const unsigned h_half = ceil_scale(height, 0.5f), h_quarter = ceil_scale(height, 0.25f);
@@ -36,7 +36,7 @@ ShardPlan compute_shard_plan(unsigned, unsigned height, const std::vector<GrbRow
 	if (bands.size() <= 1)
 	{
 		GrbRows all = { 0, (int)height };
-		p.own = p.fxaa = p.tonemap = p.lighting = all;
+		p.own = p.fxaa = p.tonemap = p.lighting = p.taa = all;
 		p.upsample0 = p.downsample0 = GrbRows{ 0, (int)h_quarter };
 		p.threshold = GrbRows{ 0, (int)h_half };
 		p.lum_grid = GrbRows{ 0, (int)h_grid };
@@ -49,7 +49,8 @@ ShardPlan compute_shard_plan(unsigned, unsigned height, const std::vector<GrbRow
 	p.downsample0 = scale_band(p.own, height, h_quarter);
 	p.threshold = clamp_rows(2 * p.downsample0.y0 - 2, 2 * p.downsample0.y1 + 2, h_half);
 	GrbRows hdr_for_threshold = clamp_rows(2 * p.threshold.y0 - 1, 2 * p.threshold.y1 + 1, height);
-	p.lighting = clamp_rows(std::min(p.tonemap.y0, hdr_for_threshold.y0), std::max(p.tonemap.y1, hdr_for_threshold.y1), height);
+	p.taa = clamp_rows(std::min(p.tonemap.y0, hdr_for_threshold.y0), std::max(p.tonemap.y1, hdr_for_threshold.y1), height);
+	p.lighting = taa ? clamp_rows(p.taa.y0 - 1, p.taa.y1 + 1, height) : p.taa;
 	// luminance grid rows: row g belongs to the rank whose band holds the first backbuffer row it maps to
 	auto begin_of = [&](unsigned r) { return (int)(((uint64_t)bands[r].y0 * h_grid + height - 1) / height); };
 	p.lum_grid.y0 = begin_of(rank);

@@ -7,6 +7,7 @@
 //   tonemap   : bloom tap = bilinear of upsample-0 at (y+0.5)/4                 -> u0 rows y/4 -+ 1
 //   d0 (1/4)  : 9-tap tent, +-1.75 texels of threshold around 2y+1 + bilinear   -> t rows 2y-2 .. 2y+3
 //   threshold : bilinear of HDR at 2y+1                                         -> HDR rows 2y .. 2y+1 (+-1)
+//   TAA       : current colour, depth and MV at +-1 row (the history is exchanged in full) -> HDR-main rows +-1
 // Bands are aligned to 64 full-res rows, so the 1/4-res d0 bands tile that level exactly.
 #pragma once
 
@@ -26,7 +27,9 @@ struct ShardPlan
 	GrbRows threshold;  // rows of "threshold" (1/2)
 	GrbRows lighting;   // rows of "HDR-main" (= rows of the G-buffer that must be resident)
 	GrbRows lum_grid;   // rows of the (d3/2) luminance grid this rank samples
+	GrbRows taa;        // rows of "HDR-resolved" (what the threshold and the tonemap read); = lighting without TAA
 };
 
-ShardPlan compute_shard_plan(unsigned width, unsigned height, const std::vector<GrbRows> &bands, unsigned rank, bool fxaa);
+// taa: a TAA resolve sits between lighting and the post chain; lighting then covers taa +-1 row.
+ShardPlan compute_shard_plan(unsigned width, unsigned height, const std::vector<GrbRows> &bands, unsigned rank, bool fxaa, bool taa = false);
 } // namespace Granite

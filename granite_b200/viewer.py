@@ -221,9 +221,15 @@ def rebalance_bands(bands, band_times, height: int, align: int = 8, damping: flo
 PLAN_FIELDS = ("own", "fxaa", "tonemap", "upsample0", "downsample0", "threshold", "lighting", "lum_grid")
 
 
-def shard_plan(width, height, bands, rank, fxaa=False) -> dict:
-    """Rows of every stage one rank computes (host math of granite_b200/host/shard_plan.cpp)."""
+def shard_plan(width, height, bands, rank, fxaa=False, taa=False) -> dict:
+    """Rows of every stage one rank computes (host math of granite_b200/host/shard_plan.cpp).  taa=True: a TAA
+    resolve precedes the post chain; the dict then also has "taa" (rows of the resolved image) and "lighting"
+    covers taa +- 1 row."""
     arr = (capi.GrbRows * max(len(bands), 1))(*[capi.GrbRows(a, b) for a, b in bands])
+    if taa:
+        out = (capi.GrbRows * 9)()
+        _check(lib().grbh_shard_plan_ex(width, height, arr, len(bands), rank, int(fxaa), 1, out), "grbh_shard_plan_ex")
+        return {k: (out[i].y0, out[i].y1) for i, k in enumerate(PLAN_FIELDS + ("taa",))}
     out = (capi.GrbRows * 8)()
     _check(lib().grbh_shard_plan(width, height, arr, len(bands), rank, int(fxaa), out), "grbh_shard_plan")
     return {k: (out[i].y0, out[i].y1) for i, k in enumerate(PLAN_FIELDS)}

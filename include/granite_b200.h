@@ -397,6 +397,19 @@ int32_t grb_fxaa(const GrbImage *in, const GrbImage *out, GrbRows rows, void *st
 int32_t grb_taa_resolve(const GrbImage *hdr, const GrbImage *depth, const GrbImage *mv,
                         const GrbImage *history, const float *reproj16, int32_t quality,
                         const GrbImage *out_color, const GrbImage *out_history, GrbRows rows, void *stream);
+/* grb_taa_resolve for one rank of a row-sharded frame, with the history exchange fused in (the exact kernel; the
+ * GRB_TAA_TILES form has no peer variant).  out_color gets the rows [rows.y0, rows.y1); the history texels of
+ * own_rows (inside rows: this rank's band) are stored into the history slot of EVERY rank -- peer_images[r], valid on
+ * this device, one of them this rank's own, all with out_history_layout's size and pitch (its data pointer is not
+ * written) -- and then peer_flags[r][flag_index] = epoch is release-stored on every rank, as in
+ * grb_bloom_downsample_to_peers.  `history` (last frame's full history) must not be one of the slots written.
+ * A raised flag also means the producing rank has finished reading its `history`.  No reference equivalent. */
+int32_t grb_taa_resolve_to_peers(const GrbImage *hdr, const GrbImage *depth, const GrbImage *mv,
+                                 const GrbImage *history, const float *reproj16, int32_t quality,
+                                 const GrbImage *out_color, const GrbImage *out_history_layout,
+                                 void *const *peer_images, uint32_t *const *peer_flags, int32_t peer_count,
+                                 int32_t flag_index, uint32_t epoch, uint32_t *scratch_counter, GrbRows rows,
+                                 GrbRows own_rows, void *stream);
 
 #ifdef __cplusplus
 }

@@ -138,6 +138,10 @@ int32_t grbh_viewer_measure_row_cost(GrbhViewer *viewer, uint32_t *out, int32_t 
 /* The row plan of one rank of a row-sharded frame (granite_b200/host/shard_plan.hpp): out8 =
  * {own, fxaa, tonemap, upsample0, downsample0, threshold, lighting, lum_grid}.  Pure host math. */
 int32_t grbh_shard_plan(int32_t width, int32_t height, const GrbRows *bands, int32_t count, int32_t rank, int32_t fxaa, GrbRows *out8);
+/* The same with a TAA resolve between lighting and the post chain (taa != 0): out9 = the eight rows above followed by
+ * taa, the rows of the resolved image (what the threshold and the tonemap read); lighting is then taa +- 1 row. */
+int32_t grbh_shard_plan_ex(int32_t width, int32_t height, const GrbRows *bands, int32_t count, int32_t rank, int32_t fxaa, int32_t taa,
+                           GrbRows *out9);
 
 /* bake_render_graph: declares the passes, bakes, allocates attachments. */
 int32_t grbh_viewer_bake(GrbhViewer *viewer);
