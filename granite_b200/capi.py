@@ -95,7 +95,7 @@ ENTRY_POINTS = [
     "grb_cluster_build", "grb_cluster_decal_binning", "grb_fog_light_density", "grb_fog_accumulate", "grb_deferred_lighting", "grb_deferred_lighting_blocks", "grb_deferred_lighting_scheduled", "grb_deferred_lighting_shadowed", "grb_lighting_schedule_bytes", "grb_debug_cluster_indices", "grb_lighting_row_cost",
     "grb_bloom_threshold", "grb_bloom_threshold_downsample", "grb_bloom_threshold_downsample_to_peers", "grb_bloom_downsample", "grb_bloom_downsample_to_peers", "grb_peer_wait", "grb_bloom_upsample", "grb_bloom_upsample_exact",
     "grb_luminance", "grb_luminance_grid", "grb_luminance_finalize", "grb_bloom_tail", "grb_bloom_tail_ex", "grb_tonemap",
-    "grb_pq10_encode", "grb_smaa_edge_detection", "grb_smaa_blend_weights", "grb_smaa_neighborhood_blend", "grb_fsr_easu_constants", "grb_fsr_upscale", "grb_fsr_sharpen", "grb_fxaa", "grb_taa_resolve", "grb_taa_resolve_to_peers",
+    "grb_pq10_encode", "grb_smaa_edge_detection", "grb_smaa_blend_weights", "grb_smaa_neighborhood_blend", "grb_smaa_edge_detection_to_peers", "grb_fsr_easu_constants", "grb_fsr_upscale", "grb_fsr_sharpen", "grb_fxaa", "grb_taa_resolve", "grb_taa_resolve_to_peers",
 ]
 
 _lib = None
@@ -147,6 +147,7 @@ def lib() -> C.CDLL:
             "grb_smaa_edge_detection": [IMG, I, IMG, GrbRows, P],
             "grb_smaa_blend_weights": [IMG, IMG, IMG, I, IMG, GrbRows, P],
             "grb_smaa_neighborhood_blend": [IMG, IMG, IMG, GrbRows, P],
+            "grb_smaa_edge_detection_to_peers": [IMG, I, IMG, P, C.POINTER(GrbRows), P, I, I, C.c_uint32, P, GrbRows, P],
             "grb_fxaa": [IMG, IMG, GrbRows, P],
             "grb_taa_resolve": [IMG, IMG, IMG, IMG, P, I, IMG, IMG, GrbRows, P],
             "grb_taa_resolve_to_peers": [IMG, IMG, IMG, IMG, P, I, IMG, IMG, P, P, I, I, C.c_uint32, P, GrbRows, GrbRows, P],

@@ -289,4 +289,29 @@ GRB_DEV float3 fetch_hdr_clamped(const View<const uint2> &im, int x, int y)
 	return hdr_texel(im, iclamp(x, 0, im.w - 1), iclamp(y, 0, im.h - 1));
 }
 
+#ifndef GRB_HOST_EMULATION
+// ---- the producing side of the peer exchanges of a row-sharded frame (bloom d0, TAA history, SMAA edges)
+GRB_DEV void store_release_system(uint32_t *p, uint32_t v) { asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory"); }
+
+// Called by every thread of every CTA after its peer stores: each thread's stores are ordered before its CTA's
+// arrival, and the last CTA to arrive resets the counter and release-stores flags[r][flag_index] = epoch on every rank r
+// (threadFenceReduction pattern at system scope).  The consumer side is grb_peer_wait.
+GRB_DEV void publish_to_peers(uint32_t *const *flags, int count, int flag_index, uint32_t epoch, unsigned *ctas_done)
+{
+	__threadfence_system();
+	__syncthreads();
+	if (threadIdx.x == 0 && threadIdx.y == 0)
+	{
+		const unsigned total = gridDim.x * gridDim.y;
+		if (atomicAdd(ctas_done, 1u) == total - 1u)
+		{
+			*ctas_done = 0u;
+			__threadfence_system();
+			for (int r = 0; r < count; r++)
+				store_release_system(flags[r] + flag_index, epoch);
+		}
+	}
+}
+#endif
+
 } // namespace grb

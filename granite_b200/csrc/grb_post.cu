@@ -132,7 +132,6 @@ struct PeerTargets
 	int count;
 };
 
-__device__ __forceinline__ void store_release_system(uint32_t *p, uint32_t v) { asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory"); }
 __device__ __forceinline__ uint32_t load_acquire_system(const uint32_t *p)
 {
 	uint32_t v;
@@ -155,21 +154,8 @@ __global__ void __launch_bounds__(kBlockX *kBlockY) bloom_downsample_peers_kerne
 		for (int r = 0; r < targets.count; r++)
 			targets.data[r][at] = texel;
 	}
-	// publish: every thread's stores are ordered before its CTA's arrival; the last CTA to arrive
-	// raises this rank's flag on every peer (threadFenceReduction pattern at system scope)
-	__threadfence_system();
-	__syncthreads();
-	if (threadIdx.x == 0 && threadIdx.y == 0)
-	{
-		const unsigned total = gridDim.x * gridDim.y;
-		if (atomicAdd(ctas_done, 1u) == total - 1u)
-		{
-			*ctas_done = 0u;
-			__threadfence_system();
-			for (int r = 0; r < targets.count; r++)
-				store_release_system(targets.flags[r] + flag_index, epoch);
-		}
-	}
+	// publish: the last CTA to arrive raises this rank's flag on every peer
+	publish_to_peers(targets.flags, targets.count, flag_index, epoch, ctas_done);
 }
 
 // One thread per producing rank spins until that rank's band of frame `epoch` has landed here.
@@ -769,22 +755,9 @@ __global__ void __launch_bounds__(kBlockX *kBlockY) taa_kernel(TaaInputsT<HdrTex
 					peers.targets.data[r][at] = texel;
 			}
 		}
-		// publish (threadFenceReduction pattern at system scope, as bloom_downsample_peers_kernel): every CTA has read
-		// its history texels and stored its band texels before it arrives, so a raised flag also says "this rank is
-		// done reading last frame's slot"
-		__threadfence_system();
-		__syncthreads();
-		if (threadIdx.x == 0 && threadIdx.y == 0)
-		{
-			const unsigned total = gridDim.x * gridDim.y;
-			if (atomicAdd(peers.ctas_done, 1u) == total - 1u)
-			{
-				*peers.ctas_done = 0u;
-				__threadfence_system();
-				for (int r = 0; r < peers.targets.count; r++)
-					store_release_system(peers.targets.flags[r] + peers.flag_index, peers.epoch);
-			}
-		}
+		// publish, as bloom_downsample_peers_kernel: every CTA has read its history texels and stored its band texels
+		// before it arrives, so a raised flag also says "this rank is done reading last frame's slot"
+		publish_to_peers(peers.targets.flags, peers.targets.count, peers.flag_index, peers.epoch, peers.ctas_done);
 	}
 }
 

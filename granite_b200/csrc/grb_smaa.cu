@@ -11,6 +11,7 @@
 // One thread per pixel.  The edge and blend passes are streaming; the weight pass returns at once for the pixels
 // without an edge (the vast majority) and walks the searches for the rest.
 #include <cstdint>
+#include <type_traits>
 
 #include "grb_common.cuh"
 
@@ -106,12 +107,55 @@ GRB_DEV uint32_t unorm8(float c)
 }
 
 // ------------------------------------------------------------------------------------------------ edges
-// SMAALumaEdgeDetectionPS (SMAA.hlsl:689-746) + SMAAEdgeDetectionVS (:645-650)
-__global__ void __launch_bounds__(256) smaa_edge_kernel(Tex8<4> col, View<uchar2> edges, SmaaPreset P, int y0, int y1)
+// The edge exchange of a row-sharded frame (the peer form of the edge pass): each edge texel of the rows [y0, y1) goes
+// to the edge slot of every rank r whose rows[r] hold its row instead of `edges`, then the last CTA raises
+// flags[flag_index] = epoch on every rank (as bloom_downsample_peers_kernel in grb_post.cu).  NoSmaaPeerStore: the
+// plain pass.  SmaaPeerStore and its two members exist only in the device build; the host emulation of this file
+// (tests/cpp/emulate_smaa.cpp) never instantiates the peer form.
+struct NoSmaaPeerStore
 {
-	const int x = blockIdx.x * 32 + threadIdx.x, y = y0 + blockIdx.y * 8 + threadIdx.y;
-	if (x >= col.w || y >= y1)
-		return;
+};
+#ifndef GRB_HOST_EMULATION
+struct SmaaPeerStore
+{
+	uchar2 *data[GRB_MAX_PEERS];
+	uint32_t *flags[GRB_MAX_PEERS];
+	int row0[GRB_MAX_PEERS], row1[GRB_MAX_PEERS];
+	int count, pitch_texels, flag_index;
+	uint32_t epoch;
+	unsigned *ctas_done;
+
+	// A warp is 32 consecutive texels of one row: each store below is 64 contiguous bytes, and the row test is
+	// uniform across the warp.
+	GRB_DEV void store(int x, int y, uchar2 v) const
+	{
+		const size_t at = (size_t)y * pitch_texels + x;
+		for (int r = 0; r < count; r++)
+			if (y >= row0[r] && y < row1[r])
+				data[r][at] = v;
+	}
+	// every CTA has stored its texels before it arrives; the last one raises the flag on every rank, also on ranks that
+	// received no rows
+	GRB_DEV void publish() const { publish_to_peers(flags, count, flag_index, epoch, ctas_done); }
+};
+#endif
+
+// SMAALumaEdgeDetectionPS (SMAA.hlsl:689-746) + SMAAEdgeDetectionVS (:645-650)
+template <typename PeerStore = NoSmaaPeerStore>
+__global__ void __launch_bounds__(256) smaa_edge_kernel(Tex8<4> col, View<uchar2> edges, SmaaPreset P, int y0, int y1, PeerStore peers = PeerStore{})
+{
+	constexpr bool kPeers = !std::is_same<PeerStore, NoSmaaPeerStore>::value;
+	int x = blockIdx.x * 32 + threadIdx.x, y = y0 + blockIdx.y * 8 + threadIdx.y;
+	const bool inside = x < col.w && y < y1;
+	if (!inside)
+	{
+		if (!kPeers)
+			return;
+		// every thread of the peer form reaches the CTA barrier of publish(): off the band it computes a clamped pixel
+		// and stores nothing
+		x = min(x, col.w - 1);
+		y = min(y, y1 - 1);
+	}
 	const float mx = fdiv(1.0f, (float)col.w), my = fdiv(1.0f, (float)col.h);
 	const Frag f = { fmul((float)x + 0.5f, mx), fmul((float)y + 0.5f, my), x, y };
 	uchar2 out = make_uchar2(0, 0);
@@ -141,7 +185,14 @@ __global__ void __launch_bounds__(256) smaa_edge_kernel(Tex8<4> col, View<uchar2
 		ey = fmul(ey, step_f(final_delta, fmul(dy, 2.0f)));
 		out = make_uchar2((unsigned char)unorm8(ex), (unsigned char)unorm8(ey));
 	}
-	edges.at(x, y) = out;
+	if constexpr (!kPeers)
+		edges.at(x, y) = out;
+	else
+	{
+		if (inside)
+			peers.store(x, y, out);
+		peers.publish();
+	}
 }
 
 // ------------------------------------------------------------------------------------------------ weights
@@ -519,6 +570,64 @@ extern "C" int32_t grb_smaa_edge_detection(const GrbImage *color, int32_t qualit
 	smaa_edge_kernel<<<smaa_grid(edges->width, rows.y1 - rows.y0), dim3(32, 8), 0, as_stream(stream)>>>(tex_of<4>(color), view_of<uchar2>(edges), preset_of(quality),
 	                                                                                                    rows.y0, rows.y1);
 	return check_launch("grb_smaa_edge_detection");
+}
+
+extern "C" int32_t grb_smaa_edge_detection_to_peers(const GrbImage *color, int32_t quality, const GrbImage *edges_layout, void *const *peer_images,
+                                                    const GrbRows *peer_rows, uint32_t *const *peer_flags, int32_t peer_count, int32_t flag_index,
+                                                    uint32_t epoch, uint32_t *scratch_counter, GrbRows rows, void *stream)
+{
+	if (!color || !edges_layout || !peer_images || !peer_rows || !peer_flags || !scratch_counter || peer_count < 1 || peer_count > GRB_MAX_PEERS ||
+	    flag_index < 0 || flag_index >= peer_count)
+	{
+		set_last_error("grb_smaa_edge_detection_to_peers: bad arguments (edges_layout, peer_images, peer_rows, peer_flags, scratch_counter; "
+		               "peer_count 1..GRB_MAX_PEERS, 0 <= flag_index < peer_count)");
+		return GRB_ERR_INVALID_ARGUMENT;
+	}
+	// the layout describes every rank's edge slot; its data pointer is not written (only the peer images are)
+	GrbImage layout = *edges_layout;
+	if (!layout.data)
+		layout.data = peer_images[0];
+	if (!rgba8(color) || !image_ok(&layout, GRB_FORMAT_R8G8_UNORM, 2) || !same_size(color, &layout) || quality < 0 || quality > 3)
+	{
+		set_last_error("grb_smaa_edge_detection_to_peers: color R8G8B8A8 (read as UNORM), edges_layout R8G8_UNORM of the same size, quality 0..3");
+		return GRB_ERR_UNSUPPORTED_FORMAT;
+	}
+	if (rows.y0 < 0 || rows.y1 <= rows.y0 || rows.y1 > color->height)
+	{
+		set_last_error("grb_smaa_edge_detection_to_peers: rows must be a non-empty range of the image (this rank's band)");
+		return GRB_ERR_INVALID_ARGUMENT;
+	}
+	if (peer_rows[flag_index].y0 != rows.y0 || peer_rows[flag_index].y1 != rows.y1)
+	{
+		set_last_error("grb_smaa_edge_detection_to_peers: peer_rows[flag_index] must equal rows (this rank's slot receives its whole band)");
+		return GRB_ERR_INVALID_ARGUMENT;
+	}
+	SmaaPeerStore peers{};
+	peers.count = peer_count;
+	for (int r = 0; r < peer_count; r++)
+	{
+		if (!peer_images[r] || !peer_flags[r])
+		{
+			set_last_error("grb_smaa_edge_detection_to_peers: null peer pointer");
+			return GRB_ERR_INVALID_ARGUMENT;
+		}
+		if (peer_rows[r].y0 > peer_rows[r].y1 || peer_rows[r].y0 < rows.y0 || peer_rows[r].y1 > rows.y1)
+		{
+			set_last_error("grb_smaa_edge_detection_to_peers: every peer_rows[r] must lie inside rows (y0 <= y1; empty: y0 == y1)");
+			return GRB_ERR_INVALID_ARGUMENT;
+		}
+		peers.data[r] = static_cast<uchar2 *>(peer_images[r]);
+		peers.flags[r] = peer_flags[r];
+		peers.row0[r] = peer_rows[r].y0;
+		peers.row1[r] = peer_rows[r].y1;
+	}
+	peers.pitch_texels = layout.row_pitch / 2;
+	peers.flag_index = flag_index;
+	peers.epoch = epoch;
+	peers.ctas_done = scratch_counter;
+	smaa_edge_kernel<SmaaPeerStore><<<smaa_grid(color->width, rows.y1 - rows.y0), dim3(32, 8), 0, as_stream(stream)>>>(tex_of<4>(color), View<uchar2>{}, preset_of(quality),
+	                                                                                                                 rows.y0, rows.y1, peers);
+	return check_launch("grb_smaa_edge_detection_to_peers");
 }
 
 extern "C" int32_t grb_smaa_blend_weights(const GrbImage *edges, const GrbImage *area, const GrbImage *search, int32_t quality, const GrbImage *weights,

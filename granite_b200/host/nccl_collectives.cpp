@@ -88,6 +88,7 @@ NcclCollectives::~NcclCollectives()
 {
 	release_peer_exchange(peer);
 	release_peer_exchange(taa_history);
+	release_peer_exchange(smaa_edges);
 	if (comm && api().CommDestroy)
 		api().CommDestroy(comm);
 }
@@ -312,5 +313,10 @@ bool NcclCollectives::taa_history_begin_frame(size_t image_bytes, PeerSlot &slot
 	if (taa_history.frames > 1)
 		previous = taa_history.local_images[(taa_history.epoch - 1) & 1u];
 	return true;
+}
+
+bool NcclCollectives::smaa_edges_begin_frame(size_t image_bytes, PeerSlot &slot)
+{
+	return begin_frame(smaa_edges, image_bytes, slot);
 }
 } // namespace Granite

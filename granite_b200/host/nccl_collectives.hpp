@@ -30,6 +30,8 @@ public:
 	bool peer_exchange_begin_frame(size_t image_bytes, PeerSlot &slot) override;
 	// The TAA history channel: a second set of the same buffers.
 	bool taa_history_begin_frame(size_t image_bytes, PeerSlot &slot, void *&previous) override;
+	// The SMAA edge channel: a third set.
+	bool smaa_edges_begin_frame(size_t image_bytes, PeerSlot &slot) override;
 
 private:
 	bool collective_failed(const char *what);
@@ -47,7 +49,7 @@ private:
 		std::vector<void *> opened;
 		uint32_t epoch = 0;
 		unsigned frames = 0; // frames begun since the buffers were (re-)created
-	} peer, taa_history;
+	} peer, taa_history, smaa_edges;
 	bool begin_frame(PeerState &peer, size_t image_bytes, PeerSlot &slot);
 	bool setup_peer_exchange(PeerState &peer, size_t image_bytes);
 	void release_peer_exchange(PeerState &peer);

@@ -5,8 +5,10 @@
 #include <cuda_runtime.h>
 
 #include <cstdio>
+#include <algorithm>
 #include <cstring>
 #include <map>
+#include <memory>
 #include <mutex>
 #include <stdexcept>
 
@@ -147,8 +149,6 @@ void setup_smaa_postprocess(RenderGraph &graph, TemporalJitter &jitter, float, c
 {
 	if (preset == SMAAPreset::Ultra_T2X)
 		throw std::logic_error("SMAA T2X (two jittered frames + smaa-t2x-resolve) is not built by this executor.");
-	if (graph.is_sharded() && graph.get_shard_count() > 1)
-		throw std::logic_error("SMAA is not available in row-sharded graphs: its searches cross band borders.");
 	const int quality = preset == SMAAPreset::Low ? 0 : (preset == SMAAPreset::Medium ? 1 : (preset == SMAAPreset::High ? 2 : 3));
 	jitter.init(TemporalJitter::Type::None, vec2(1.0f)); // smaa.cpp:66-67
 
@@ -179,12 +179,56 @@ void setup_smaa_postprocess(RenderGraph &graph, TemporalJitter &jitter, float, c
 	auto &blend_input = smaa_blend.add_texture_input(input);
 	auto &blend_weights = smaa_blend.add_texture_input("smaa-weights");
 
-	smaa_edge.set_build_render_pass([&graph, &edge_out, &edge_input, quality](Vulkan::CommandBuffer &cmd) {
+	// Row-sharded frames (graph.get_shard_plan(): smaa_weights, smaa_edges): the weights pass of a rank walks edges up to
+	// 2 * max_search_steps + 4 rows beyond its band, so the edges are exchanged rather than recomputed.  Each rank
+	// detects the edges of its own band only; on the peer path "smaa-edge" stores every edge row into the slot of each
+	// rank whose window (plan.smaa_edges) holds it and raises a flag on every rank, and "smaa-weights" waits for every
+	// rank's flag of this frame, then reads this rank's slot.  Two slots suffice: the three passes share one stream (the
+	// post-graphics queue), so a rank's frame N+1 edge pass runs after its frame N weights pass, which waited for every
+	// rank's frame-N flag; each of those was raised after that rank's frame N-1 weights pass, the last reader of slot
+	// (N+1) mod 2.  On the NCCL path "smaa-edge" writes the band into the graph's image and all-gathers the bands.
+	// `edges_slot` carries this frame's slot from the edge pass to the weights pass (both record on this thread, in order).
+	auto edges_slot = std::make_shared<RenderGraphCollectives::PeerSlot>();
+	auto sharded = [&graph] { return graph.is_sharded() && graph.get_shard_count() > 1; };
+	smaa_edge.set_build_render_pass([&graph, &edge_out, &edge_input, quality, edges_slot, sharded](Vulkan::CommandBuffer &cmd) {
 		GrbImage color = graph.get_physical_texture_resource(edge_input).as_grb_unorm();
 		GrbImage edges = graph.get_physical_texture_resource(edge_out).as_grb();
-		cmd.check(grb_smaa_edge_detection(&color, quality, &edges, GrbRows{ 0, 0 }, cmd.get_stream_handle()), "grb_smaa_edge_detection");
+		*edges_slot = RenderGraphCollectives::PeerSlot{};
+		if (!sharded())
+		{
+			cmd.check(grb_smaa_edge_detection(&color, quality, &edges, GrbRows{ 0, 0 }, cmd.get_stream_handle()), "grb_smaa_edge_detection");
+			return;
+		}
+		const ShardPlan plan = graph.get_shard_plan();
+		auto *collectives = graph.get_collectives();
+		const unsigned self = collectives->get_rank(), count = graph.get_shard_count();
+		RenderGraphCollectives::PeerSlot slot;
+		if (collectives->smaa_edges_begin_frame((size_t)edges.row_pitch * (size_t)edges.height, slot))
+		{
+			// rank r receives the rows of this band its window holds (own ∩ smaa_edges of r; empty: y0 == y1)
+			GrbRows peer_rows[GRB_MAX_PEERS] = {};
+			for (unsigned r = 0; r < count; r++)
+			{
+				const GrbRows window = graph.get_shard_plan(r).smaa_edges;
+				const int y0 = std::max(plan.own.y0, window.y0), y1 = std::min(plan.own.y1, window.y1);
+				peer_rows[r] = y0 < y1 ? GrbRows{ y0, y1 } : GrbRows{ plan.own.y0, plan.own.y0 };
+			}
+			GrbImage layout = edges;
+			layout.data = nullptr;
+			cmd.check(grb_smaa_edge_detection_to_peers(&color, quality, &layout, slot.images, peer_rows, slot.flags, (int32_t)slot.count, (int32_t)self,
+			                                           slot.epoch, slot.counter, plan.own, cmd.get_stream_handle()),
+			          "grb_smaa_edge_detection_to_peers");
+			*edges_slot = slot;
+			return;
+		}
+		// NCCL path: this band into the graph's image, then every rank broadcasts its band
+		cmd.check(grb_smaa_edge_detection(&color, quality, &edges, plan.own, cmd.get_stream_handle()), "grb_smaa_edge_detection");
+		std::vector<GrbRows> bands;
+		for (unsigned r = 0; r < count; r++)
+			bands.push_back(graph.get_shard_plan(r).own);
+		collectives->all_gather_rows(cmd, graph.get_physical_texture_resource(edge_out), bands);
 	});
-	smaa_weight.set_build_render_pass([&graph, &weight_out, &weight_input, quality](Vulkan::CommandBuffer &cmd) {
+	smaa_weight.set_build_render_pass([&graph, &weight_out, &weight_input, quality, edges_slot, sharded](Vulkan::CommandBuffer &cmd) {
 		GrbImage edges = graph.get_physical_texture_resource(weight_input).as_grb();
 		GrbImage weights = graph.get_physical_texture_resource(weight_out).as_grb();
 		GrbImage area, search;
@@ -193,13 +237,27 @@ void setup_smaa_postprocess(RenderGraph &graph, TemporalJitter &jitter, float, c
 			Vulkan::log_error("smaa-weights: no lookup textures on this device (set_smaa_lookup_textures / load_smaa_lookup_textures).\n");
 			return;
 		}
-		cmd.check(grb_smaa_blend_weights(&edges, &area, &search, quality, &weights, GrbRows{ 0, 0 }, cmd.get_stream_handle()), "grb_smaa_blend_weights");
+		GrbRows rows = GrbRows{ 0, 0 };
+		if (sharded())
+		{
+			rows = graph.get_shard_plan().smaa_weights;
+			if (edges_slot->count)
+			{
+				// peer path: every rank's edges of this frame have arrived in this rank's slot
+				const unsigned self = graph.get_collectives()->get_rank();
+				cmd.check(grb_peer_wait(edges_slot->flags[self], (int32_t)edges_slot->count, edges_slot->epoch, cmd.get_stream_handle()),
+				          "grb_peer_wait(smaa edges)");
+				edges.data = edges_slot->images[self];
+			}
+		}
+		cmd.check(grb_smaa_blend_weights(&edges, &area, &search, quality, &weights, rows, cmd.get_stream_handle()), "grb_smaa_blend_weights");
 	});
-	smaa_blend.set_build_render_pass([&graph, &blend_out, &blend_input, &blend_weights](Vulkan::CommandBuffer &cmd) {
+	smaa_blend.set_build_render_pass([&graph, &blend_out, &blend_input, &blend_weights, sharded](Vulkan::CommandBuffer &cmd) {
 		GrbImage color = graph.get_physical_texture_resource(blend_input).as_grb_unorm();
 		GrbImage weights = graph.get_physical_texture_resource(blend_weights).as_grb();
 		GrbImage out = graph.get_physical_texture_resource(blend_out).as_grb(); // SMAA_TARGET_SRGB follows the output format (smaa.cpp:193-194)
-		cmd.check(grb_smaa_neighborhood_blend(&color, &weights, &out, GrbRows{ 0, 0 }, cmd.get_stream_handle()), "grb_smaa_neighborhood_blend");
+		const GrbRows rows = sharded() ? graph.get_shard_plan().own : GrbRows{ 0, 0 };
+		cmd.check(grb_smaa_neighborhood_blend(&color, &weights, &out, rows, cmd.get_stream_handle()), "grb_smaa_neighborhood_blend");
 	});
 }
 } // namespace Granite

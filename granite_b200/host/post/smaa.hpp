@@ -21,8 +21,9 @@ enum class SMAAPreset
 
 // Three passes on the post-graphics queue -- "smaa-edge" (R8G8_UNORM), "smaa-weights" (R8G8B8A8_UNORM), "smaa-blend" --
 // reading `input` (the tonemapped image, viewed as UNORM) and writing `output` (renderer/post/smaa.cpp:32-209).
-// Ultra_T2X (two jittered frames + "smaa-t2x-resolve") is not built: std::logic_error.  Not available in row-sharded
-// graphs (the searches reach up to 64 pixels across a band's border): std::logic_error as well.
+// Ultra_T2X (two jittered frames + "smaa-t2x-resolve") is not built: std::logic_error.  In row-sharded graphs each rank
+// detects the edges of its band, the edge rows another rank's searches reach are exchanged (peer stores from the edge
+// kernel, or NCCL broadcasts), and each rank computes the weights of ShardPlan::smaa_weights and blends its band.
 void setup_smaa_postprocess(RenderGraph &graph, TemporalJitter &jitter, float scaling_factor, const std::string &input, const std::string &input_depth,
                             const std::string &output, SMAAPreset preset);
 

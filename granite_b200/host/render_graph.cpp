@@ -775,10 +775,11 @@ void RenderGraph::log()
 }
 
 void RenderGraph::set_row_shards(const std::vector<GrbRows> &bands, unsigned rank, RenderGraphCollectives *collectives_, bool fxaa_downstream,
-                                 bool taa_upstream)
+                                 bool taa_upstream, int smaa_quality)
 {
 	shard_fxaa = fxaa_downstream;
 	shard_taa = taa_upstream;
+	shard_smaa = smaa_quality;
 	if (!bands.empty())
 	{
 		if (rank >= bands.size())

@@ -81,6 +81,15 @@ public:
 		previous = nullptr;
 		return false;
 	}
+	// A third channel of the same kind for the SMAA edges: each rank stores the edge rows of its band that another
+	// rank's weights pass reads into that rank's slot (slot.images[get_rank()] is this rank's own copy, which its
+	// weights pass reads).  false = not available: callers then use all_gather_rows().
+	virtual bool smaa_edges_begin_frame(size_t image_bytes, PeerSlot &slot)
+	{
+		(void)image_bytes;
+		(void)slot;
+		return false;
+	}
 };
 
 class RenderPassInterface
@@ -472,13 +481,14 @@ public:
 	// Row-sharded frames (multi-GPU, one graph per device/process): `bands[r]` = backbuffer rows
 	// [y0, y1) owned by rank r; they must tile the frame.  Builders scale the local band per
 	// resource with shard_rows_for(); an unsharded graph returns {0,0} (= all rows).
+	// smaa_quality: SMAA (0..3) after the tonemap, -1 = none (ShardPlan::smaa_weights / smaa_edges).
 	void set_row_shards(const std::vector<GrbRows> &bands, unsigned rank, RenderGraphCollectives *collectives, bool fxaa_downstream = false,
-	                    bool taa_upstream = false);
+	                    bool taa_upstream = false, int smaa_quality = -1);
 	// Rows of every stage for `rank` (this rank by default); whole images when unsharded.
 	ShardPlan get_shard_plan() const { return get_shard_plan(shard_rank); }
 	ShardPlan get_shard_plan(unsigned rank) const
 	{
-		return compute_shard_plan(swapchain_dimensions.width, swapchain_dimensions.height, shard_bands, rank, shard_fxaa, shard_taa);
+		return compute_shard_plan(swapchain_dimensions.width, swapchain_dimensions.height, shard_bands, rank, shard_fxaa, shard_taa, shard_smaa);
 	}
 	GrbRows shard_rows_for(unsigned resource_height, unsigned halo_rows = 0) const;
 	GrbRows shard_rows_for_rank(unsigned rank, unsigned resource_height, unsigned halo_rows = 0) const;
@@ -540,6 +550,7 @@ private:
 	unsigned shard_rank = 0;
 	bool shard_fxaa = false;
 	bool shard_taa = false;
+	int shard_smaa = -1;
 	RenderGraphCollectives *collectives = nullptr;
 
 	RenderTextureResource &get_or_create_texture(const std::string &name);

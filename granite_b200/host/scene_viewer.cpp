@@ -88,12 +88,13 @@ struct GrbhViewer
 	int render_height() const { return upscales() ? std::max(int(std::ceil(config.resolution_scale * float(config.height))), 1) : config.height; }
 	bool uses_fxaa() const { return config.post_aa == GRBH_AA_FXAA || config.post_aa == GRBH_AA_TAA_HIGH_PLUS_FXAA; }
 	bool uses_smaa() const { return config.post_aa >= GRBH_AA_SMAA_LOW && config.post_aa <= GRBH_AA_SMAA_ULTRA; }
+	int smaa_quality() const { return uses_smaa() ? config.post_aa - GRBH_AA_SMAA_LOW : -1; }
 
 	// rows of the full-resolution inputs this rank must hold: its band + the halo the bloom
-	// threshold (and FXAA through the tonemap, and the TAA resolve) reaches into
+	// threshold (and FXAA or SMAA through the tonemap, and the TAA resolve) reaches into
 	GrbRows input_rows() const
 	{
-		return compute_shard_plan((unsigned)render_width(), (unsigned)render_height(), bands, rank, uses_fxaa(), uses_taa()).lighting;
+		return compute_shard_plan((unsigned)render_width(), (unsigned)render_height(), bands, rank, uses_fxaa(), uses_taa(), smaa_quality()).lighting;
 	}
 
 	void upload_rows(Vulkan::CommandBuffer &cmd, RenderTextureResource *res, const void *host, unsigned texel)
@@ -126,7 +127,7 @@ void GrbhViewer::bake_render_graph()
 	dim.format = VK_FORMAT_R8G8B8A8_SRGB; // headless swapchain format (application_headless.cpp:207)
 	graph.set_backbuffer_dimensions(dim);
 	if (!bands.empty())
-		graph.set_row_shards(bands, rank, collectives.get(), uses_fxaa(), uses_taa());
+		graph.set_row_shards(bands, rank, collectives.get(), uses_fxaa(), uses_taa(), smaa_quality());
 
 	// scene.add_render_passes(graph) -> LightClusterer::add_render_passes
 	cluster.set_resolution((unsigned)config.cluster_res[0], (unsigned)config.cluster_res[1], (unsigned)config.cluster_res[2]);
@@ -677,6 +678,21 @@ extern "C" int32_t grbh_shard_plan_ex(int32_t width, int32_t height, const GrbRo
 	const GrbRows all[9] = { p.own, p.fxaa, p.tonemap, p.upsample0, p.downsample0, p.threshold, p.lighting, p.lum_grid, p.taa };
 	for (int i = 0; i < 9; i++)
 		out9[i] = all[i];
+	return 0;
+	GRBH_CATCH
+}
+
+extern "C" int32_t grbh_shard_plan_smaa(int32_t width, int32_t height, const GrbRows *bands, int32_t count, int32_t rank, int32_t fxaa, int32_t taa,
+                                        int32_t smaa_quality, GrbRows *out11)
+{
+	if (width <= 0 || height <= 0 || count < 0 || (count && !bands) || !out11 || (count && (rank < 0 || rank >= count)) || smaa_quality > 3)
+		return fail("grbh_shard_plan_smaa: bad arguments");
+	GRBH_TRY
+	std::vector<GrbRows> b(bands, bands + count);
+	ShardPlan p = compute_shard_plan((unsigned)width, (unsigned)height, b, (unsigned)rank, fxaa != 0, taa != 0, smaa_quality < 0 ? -1 : smaa_quality);
+	const GrbRows all[11] = { p.own, p.fxaa, p.tonemap, p.upsample0, p.downsample0, p.threshold, p.lighting, p.lum_grid, p.taa, p.smaa_weights, p.smaa_edges };
+	for (int i = 0; i < 11; i++)
+		out11[i] = all[i];
 	return 0;
 	GRBH_CATCH
 }

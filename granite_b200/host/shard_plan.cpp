@@ -28,7 +28,15 @@ GrbRows scale_band(GrbRows band, unsigned from_h, unsigned to_h)
 }
 } // namespace
 
-ShardPlan compute_shard_plan(unsigned, unsigned height, const std::vector<GrbRows> &bands, unsigned rank, bool fxaa, bool taa)
+void smaa_edge_reach(int quality, int &up, int &down)
+{
+	static const int max_search_steps[4] = { 4, 8, 16, 32 }; // SMAA.hlsl:304-324, grb_smaa.cu preset_of()
+	const int s = max_search_steps[quality < 0 ? 0 : (quality > 3 ? 3 : quality)];
+	up = 2 * s + 2;
+	down = 2 * s + 4;
+}
+
+ShardPlan compute_shard_plan(unsigned, unsigned height, const std::vector<GrbRows> &bands, unsigned rank, bool fxaa, bool taa, int smaa_quality)
 {
 	ShardPlan p = {};
 	const unsigned h_half = ceil_scale(height, 0.5f), h_quarter = ceil_scale(height, 0.25f);
@@ -36,7 +44,7 @@ ShardPlan compute_shard_plan(unsigned, unsigned height, const std::vector<GrbRow
 	if (bands.size() <= 1)
 	{
 		GrbRows all = { 0, (int)height };
-		p.own = p.fxaa = p.tonemap = p.lighting = p.taa = all;
+		p.own = p.fxaa = p.tonemap = p.lighting = p.taa = p.smaa_weights = p.smaa_edges = all;
 		p.upsample0 = p.downsample0 = GrbRows{ 0, (int)h_quarter };
 		p.threshold = GrbRows{ 0, (int)h_half };
 		p.lum_grid = GrbRows{ 0, (int)h_grid };
@@ -45,6 +53,15 @@ ShardPlan compute_shard_plan(unsigned, unsigned height, const std::vector<GrbRow
 	p.own = bands[rank];
 	p.fxaa = p.own;
 	p.tonemap = fxaa ? clamp_rows(p.own.y0 - 6, p.own.y1 + 6, height) : p.own;
+	p.smaa_weights = p.smaa_edges = p.own;
+	if (smaa_quality >= 0)
+	{
+		int up = 0, down = 0;
+		smaa_edge_reach(smaa_quality, up, down);
+		p.tonemap = clamp_rows(p.own.y0 - 3, p.own.y1 + 2, height);
+		p.smaa_weights = clamp_rows(p.own.y0 - 1, p.own.y1 + 2, height);
+		p.smaa_edges = clamp_rows(p.smaa_weights.y0 - up, p.smaa_weights.y1 + down, height);
+	}
 	p.upsample0 = clamp_rows(p.tonemap.y0 / 4 - 1, (p.tonemap.y1 + 3) / 4 + 1, h_quarter);
 	p.downsample0 = scale_band(p.own, height, h_quarter);
 	p.threshold = clamp_rows(2 * p.downsample0.y0 - 2, 2 * p.downsample0.y1 + 2, h_half);

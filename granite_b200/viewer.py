@@ -221,11 +221,18 @@ def rebalance_bands(bands, band_times, height: int, align: int = 8, damping: flo
 PLAN_FIELDS = ("own", "fxaa", "tonemap", "upsample0", "downsample0", "threshold", "lighting", "lum_grid")
 
 
-def shard_plan(width, height, bands, rank, fxaa=False, taa=False) -> dict:
+def shard_plan(width, height, bands, rank, fxaa=False, taa=False, smaa=None) -> dict:
     """Rows of every stage one rank computes (host math of granite_b200/host/shard_plan.cpp).  taa=True: a TAA
     resolve precedes the post chain; the dict then also has "taa" (rows of the resolved image) and "lighting"
-    covers taa +- 1 row."""
+    covers taa +- 1 row.  smaa=0..3 (Low .. Ultra): SMAA follows the tonemap; the dict then also has "smaa_weights"
+    (rows of the weights a rank computes) and "smaa_edges" (rows of the edges its weights pass reads), and
+    "tonemap" covers own - 3 .. own + 2."""
     arr = (capi.GrbRows * max(len(bands), 1))(*[capi.GrbRows(a, b) for a, b in bands])
+    if smaa is not None:
+        out = (capi.GrbRows * 11)()
+        _check(lib().grbh_shard_plan_smaa(width, height, arr, len(bands), rank, int(fxaa), int(taa), int(smaa), out), "grbh_shard_plan_smaa")
+        names = PLAN_FIELDS + ("taa", "smaa_weights", "smaa_edges")
+        return {k: (out[i].y0, out[i].y1) for i, k in enumerate(names) if k != "taa" or taa}
     if taa:
         out = (capi.GrbRows * 9)()
         _check(lib().grbh_shard_plan_ex(width, height, arr, len(bands), rank, int(fxaa), 1, out), "grbh_shard_plan_ex")

@@ -374,6 +374,15 @@ int32_t grb_smaa_edge_detection(const GrbImage *color, int32_t quality, const Gr
 int32_t grb_smaa_blend_weights(const GrbImage *edges, const GrbImage *area, const GrbImage *search, int32_t quality,
                                const GrbImage *weights, GrbRows rows, void *stream);
 int32_t grb_smaa_neighborhood_blend(const GrbImage *color, const GrbImage *weights, const GrbImage *out, GrbRows rows, void *stream);
+/* grb_smaa_edge_detection for one rank of a row-sharded frame, with the edge exchange fused in.  The edges of `rows` (this
+ * rank's band) are computed once; each texel of row y is stored into the edge slot of every rank r with y in
+ * peer_rows[r] -- peer_images[r], valid on this device, all with edges_layout's size and pitch (its data pointer is not
+ * written) -- and then peer_flags[r][flag_index] = epoch is release-stored on EVERY rank, also on ranks that received
+ * no rows, as in grb_bloom_downsample_to_peers.  peer_rows[flag_index] (this rank's own slot) must equal rows; every
+ * peer_rows[r] must lie inside rows (empty: y0 == y1).  Launches nothing on a bad argument.  No reference equivalent. */
+int32_t grb_smaa_edge_detection_to_peers(const GrbImage *color, int32_t quality, const GrbImage *edges_layout, void *const *peer_images,
+                                         const GrbRows *peer_rows, uint32_t *const *peer_flags, int32_t peer_count, int32_t flag_index,
+                                         uint32_t epoch, uint32_t *scratch_counter, GrbRows rows, void *stream);
 
 /* FidelityFX FSR 1 after the post chain (renderer/post/aa.cpp:75-174 setup_after_post_chain_upscaling;
  * assets/shaders/post/ffx-fsr/{upscale,sharpen}.frag over ffx_fsr1.h, 32-bit paths).

@@ -142,6 +142,12 @@ int32_t grbh_shard_plan(int32_t width, int32_t height, const GrbRows *bands, int
  * taa, the rows of the resolved image (what the threshold and the tonemap read); lighting is then taa +- 1 row. */
 int32_t grbh_shard_plan_ex(int32_t width, int32_t height, const GrbRows *bands, int32_t count, int32_t rank, int32_t fxaa, int32_t taa,
                            GrbRows *out9);
+/* The same with SMAA after the tonemap (smaa_quality 0..3 = Low .. Ultra; < 0: no SMAA, then out11 = out9 of
+ * grbh_shard_plan_ex with smaa_weights = smaa_edges = own): out11 = the nine rows above followed by smaa_weights (the
+ * rows of "smaa-weights" a rank computes: what its blend reads, own - 1 .. own + 2) and smaa_edges (the rows of "smaa-edge" its weights
+ * pass reads: the window its neighbours store into its edge slot).  With SMAA the tonemap covers own - 3 .. own + 2. */
+int32_t grbh_shard_plan_smaa(int32_t width, int32_t height, const GrbRows *bands, int32_t count, int32_t rank, int32_t fxaa, int32_t taa,
+                             int32_t smaa_quality, GrbRows *out11);
 
 /* bake_render_graph: declares the passes, bakes, allocates attachments. */
 int32_t grbh_viewer_bake(GrbhViewer *viewer);
